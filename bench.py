@@ -5,7 +5,7 @@ BASELINE config as a sub-record (`configs`): C3 (6 x Radial, forward + inverse),
 the ranks), C5 (RealNVP logpdf, N=2^22 TOTAL sharded, ending in the path's ONE collective, b2b_allreduce_sum_f64,
 INSIDE the timed region), each with an in-run oracle check on a 1024-column sample.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Prints ONE JSON line (rank 0).
   value      whole-job samples/s with the batch resident in HBM (CUDA events, max over ranks)
@@ -13,6 +13,8 @@ A "step" is one pass of the hot path over one batch of synthetic input.  Prints 
   roofline   dominant kernel (the fused chain kernel): algorithmic bytes per launch / measured launch time
   cpu_baseline  the C restatement of the reference CPU path (oracle/b2b_oracle.c) on the host cores
   configs    sub-records of the other BASELINE configs (same timing rules: CUDA events, max over ranks, >= 3 warm-ups)
+--dump-outputs DIR also writes what the last timed headline step returned (see dump_outputs), so that two builds can be
+compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -32,6 +34,7 @@ D, NCOLS, NLAYERS = 128, 1 << 20, 8
 METRIC = "samples/sec: with_logabsdet_jacobian through 8-layer Planar flow, D=128"
 WORKLOAD = "Composed(8x PlanarLayer), D=128, N=2^20 per GPU, Float32 (BASELINE configs[1])"
 CPU_SAMPLE_COLS = 1 << 18  # per step of the --impl reference arm
+DUMP_COLS = 1 << 16  # columns of y that --dump-outputs writes: D x 2^16 Float32 = 32 MiB (+ 4 MiB of logjac)
 f32 = np.float32
 
 
@@ -45,6 +48,18 @@ def planar_params(seed_base=100):
         b = rng.standard_normal(1).astype(np.float32)
         out.append((w, u, b))
     return out
+
+
+def dump_outputs(out_dir, y, lj):
+    """What a caller of the timed path receives from with_logabsdet_jacobian(flow, x), as Float32 .npy files:
+    DIR/logjac.npy, all N values, and DIR/y.npy, the (D, DUMP_COLS) columns of y at the sorted indices
+    np.sort(default_rng(0).choice(N, DUMP_COLS, replace=False)) -- y itself is 512 MiB."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    cols = torch.as_tensor(np.sort(np.random.default_rng(0).choice(NCOLS, DUMP_COLS, replace=False)), device=y.device)
+    np.save(os.path.join(out_dir, "y.npy"), np.ascontiguousarray(y[:, cols].cpu().numpy(), dtype=f32))
+    np.save(os.path.join(out_dir, "logjac.npy"), np.ascontiguousarray(lj.cpu().numpy(), dtype=f32))
 
 
 def measured_peaks():
@@ -383,7 +398,13 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--profile", action="store_true",
                     help="profiling runs (under ncu): only the warm-up and the timed headline steps, no JSON contract line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write y and logjac of the last timed headline step to DIR/*.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path; --impl reference has other inputs")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -455,6 +476,8 @@ def main():
     ms_total = float(ms)
     clocks = sampler.stop() if sampler else None
     value = world * NCOLS * steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y, lj)
 
     if args.profile:
         if rank == 0:
